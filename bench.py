@@ -1,7 +1,7 @@
 """bench.py — the hot path's headline benchmark (BASELINE.json: prefill attn TFLOP/s & paged-decode
 KV GB/s at 1/2/4/8 B200, % of roofline).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 A "step" is one pass of the hot path over one batch of synthetic input.
 
@@ -46,6 +46,7 @@ C2 = dict(B=4, Hq=32, Hkv=8, N=8192, D=128)
 C3 = dict(B=64, Hq=32, Hkv=8, L=4096, D=128, bs=16)
 C4 = dict(B=1, Hq=32, Hkv=8, N=65536, D=128)
 CPU_DECODE_SAMPLE = dict(B=16, Hq=32, Hkv=8, L=4096, D=128, bs=16)
+DUMP_ROWS = 512          # token rows of O that --dump-outputs writes: (4, 32, 512, 128) float32 = 32 MiB of the 512 MiB tensor
 
 _JSON_FD = None
 
@@ -102,6 +103,16 @@ def c4_config(n_gpus: int):
             "global_batch": 1, "seq_len": C4["N"], "heads": f"{C4['Hq']}q/{C4['Hkv']}kv", "head_dim": C4["D"], "causal": True,
             "parallelism": f"kv-head groups x{n_gpus} ({C4['Hkv'] // n_gpus} per GPU) + fused NVLink all-gather of O",
             "l2_policy": "inputs and the 512 MiB output are larger than L2"}
+
+
+def dump_outputs(torch, out_dir: str, o):
+    """--dump-outputs: O of the last timed C2 step as `<out_dir>/o.npy` in float32, restricted to DUMP_ROWS token rows
+    (every batch, head and column of each) drawn with a fixed seed, so that two builds run with the same arguments can be
+    compared output for output."""
+    import numpy as np
+    rows = torch.randperm(o.shape[2], generator=torch.Generator().manual_seed(0xC0FFEE + 8))[:DUMP_ROWS].sort().values
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "o.npy"), o.index_select(2, rows.to(o.device)).float().cpu().numpy())
 
 
 def decode_bytes(B, Hq, Hkv, L, D, bs, elt=2):
@@ -731,9 +742,15 @@ def main():
     ap.add_argument("--no-sustained", action="store_true")
     ap.add_argument("--no-strong", action="store_true")
     ap.add_argument("--no-shapes", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the output of the last one as DIR/<name>.npy (float32, seeded sample)")
     ap.add_argument("--cpu-child", default=None, choices=["prefill", "decode"], help=argparse.SUPPRESS)
     ap.add_argument("--cpu-passes", type=int, default=3, help=argparse.SUPPRESS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to the GPU arm (--impl b200)")
     if args.cpu_child:
         cpu_child_main(args.cpu_child, args.cpu_passes)
         return
@@ -751,6 +768,8 @@ def main():
 
     import physics_llm_inference_b200 as pli
 
+    if args.dump_outputs and world > 1:
+        raise SystemExit("--dump-outputs writes the one-GPU C2 output; run it with --gpus 1")
     rank, world, local = pli.init_distributed("nccl" if world > 1 else None)
     assert torch.cuda.is_available(), "bench.py needs a CUDA device (there is no CPU fallback)"
     torch.cuda.set_device(local)
@@ -770,7 +789,10 @@ def main():
     torch.cuda.synchronize()
     flops_step = pli.prefill_algorithmic_flops(c["B"], c["Hq"], c["N"], c["N"], c["D"], True)
     assert pli.prefill_kernel_kind(q, k, v) == "tcgen05"
-    c2_step = lambda: pli.flash_attention_forward(q, k, v, causal=True)  # noqa: E731
+    last = {}
+
+    def c2_step():
+        last["o"] = pli.flash_attention_forward(q, k, v, causal=True)
 
     # ---- C2 device-resident timing: W warm-ups, exactly K steps between events (the headline at N = 1; `weak_c2` at N > 1,
     #      where a handful of steps is enough) ----
@@ -782,6 +804,8 @@ def main():
         ms_step = T.timed(c2_step, 0, c2_steps)
     launches = pli.launch_count()
     value = flops_step * world / (ms_step * 1e-3) / 1e12
+    if args.dump_outputs:
+        dump_outputs(torch, args.dump_outputs, last["o"])
 
     if world > 1:
         # ================= N > 1: the partitioned workload (C4, strong scaling, fused all-gather) is the headline =================

@@ -1,5 +1,5 @@
 import os, sys, time
-sys.path.insert(0, "/root/repo")
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 import physics_llm_inference_b200 as pli
 B, Hq, Hkv, L, D, bs = 256, 4, 1, 1024, 128, 16
