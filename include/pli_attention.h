@@ -177,6 +177,33 @@ int pli_decode_fwd(const void* q, const void* k_store, const void* v_store,
 int pli_decode_kernel_kind(int D, int dtype, int block_size, const int64_t kv_strides[4],
                            const void* k_store, const void* v_store);
 
+/* Decode with q_len (1..16) new query tokens per sequence in ONE split-KV launch: the verify step of speculative
+ * decoding, multi-token-prediction heads, short chunk tails.  Maths: ch02/cached_generation.py:72-94 for seq_len = q_len
+ * > 1, with the offset causal mask :85-91: query i of sequence b sees key j iff j <= i + seq_lens[b] - q_len.
+ *   q (B,Hq,q_len,D) with strides {batch, head, token}, any (e.g. the (B,q_len,Hq,D).transpose(1,2) view of a projection);
+ *   o (B,Hq,q_len,D) with strides {batch, head, token}: its head stride must be q_len * its token stride (a tensor
+ *   contiguous in its last three dimensions; PLI_ERR_INVALID otherwise);  lse (B,Hq,q_len) f32 contiguous or NULL;
+ *   seq_lens (B,) int32 device: cached length INCLUDING the q_len new tokens (their K/V already appended, as for
+ *   pli_prefill_paged_fwd); requires seq_lens[b] >= q_len (not checked on the device).
+ *   Other arguments as for pli_decode_fwd.  The q_len rows of a q head are served as extra rows of its KV group (G*q_len
+ *   rows per KV head, in 16-row chunks), so each K/V byte is still read once per chunk;
+ *   workspace: pli_decode_workspace_bytes(B, Hq*q_len, D, num_splits);
+ *   num_splits = 0 picks pli_decode_num_splits_multi(B, Hq, Hkv, q_len, max_seq_len).
+ * q_len > 16: PLI_ERR_UNSUPPORTED (use pli_prefill_paged_fwd / pli_prefill_fwd).  The peer-output entries above take one
+ * token per sequence.  With q_len = 1 this computes what pli_decode_fwd computes, with the same automatic split count. */
+int pli_decode_fwd_multi(const void* q, const void* k_store, const void* v_store,
+                         const int32_t* block_table, const int32_t* seq_lens,
+                         void* o, float* lse,
+                         int B, int Hq, int Hkv, int q_len, int D, int max_seq_len,
+                         int block_size, int table_stride, int layer, int64_t kv_extent,
+                         const int64_t q_strides[3], const int64_t kv_strides[4], const int64_t o_strides[3],
+                         float scale, int dtype, int num_splits,
+                         void* workspace, size_t workspace_bytes, void* stream);
+/* The split count pli_decode_fwd_multi picks for num_splits = 0: its grid's units are (b, kv head, 16-row chunk of the
+ * G*q_len rows of a KV head), i.e. pli_decode_num_splits(B, Hkv*ceil(G*q_len/16), max_seq_len); for q_len = 1 exactly
+ * pli_decode_num_splits(B, Hkv, max_seq_len). */
+int pli_decode_num_splits_multi(int B, int Hq, int Hkv, int q_len, int max_seq_len);
+
 /* Decode fused with the all-gather of its output over NVLink / NVSwitch peer memory.  The reference has no
  * collective (ch09/nccl_primitives.py:45-67 only models all-gather cost); a tensor-parallel caller that shards KV
  * heads over ranks (one process per GPU) needs every rank's heads on every rank after the attention block.  Here

@@ -48,6 +48,7 @@ _SIGNATURES = {
                                                _I64P, _I64P, C.c_float, C.c_int, _VP]),
     "pli_prefill_kernel_kind": (C.c_int, [C.c_int, C.c_int, _I64P, _I64P, _I64P, _I64P, _VP, _VP, _VP, _VP]),
     "pli_decode_num_splits": (C.c_int, [C.c_int, C.c_int, C.c_int]),
+    "pli_decode_num_splits_multi": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int, C.c_int]),
     "pli_decode_workspace_bytes": (C.c_size_t, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "pli_decode_splitkv": (C.c_int, [_VP, _VP, _VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                      C.c_int, C.c_int, C.c_int64, _I64P, _I64P, C.c_float, C.c_int, C.c_int, _VP,
@@ -56,6 +57,9 @@ _SIGNATURES = {
     "pli_decode_fwd": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                  C.c_int, C.c_int, C.c_int, C.c_int64, _I64P, _I64P, _I64P, C.c_float, C.c_int,
                                  C.c_int, _VP, C.c_size_t, _VP]),
+    "pli_decode_fwd_multi": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
+                                       C.c_int, C.c_int, C.c_int, C.c_int, C.c_int64, _I64P, _I64P, _I64P, C.c_float,
+                                       C.c_int, C.c_int, _VP, C.c_size_t, _VP]),
     "pli_decode_kernel_kind": (C.c_int, [C.c_int, C.c_int, C.c_int, _I64P, _VP, _VP]),
     "pli_decode_fwd_scatter": (C.c_int, [_VP, _VP, _VP, _VP, _VP, _VP, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int,
                                          C.c_int, C.c_int, C.c_int, C.c_int64, _I64P, _I64P, _I64P, C.c_float, C.c_int,

@@ -2,8 +2,9 @@
 // the KV append (write path), the page-gather parity aid and the NVLink gather of the output.
 //
 // Maths: ch02/cached_generation.py:72-94 for seq_len == 1 (no mask, :85) with the GQA map of
-// :77-78.  Addressing: ch07/paged_memory.py:38-48 pool layout, token t -> page table[t / bs],
-// slot t % bs (ceil-div rule, :54,:84-86).  HBM-bound: each K/V byte is read exactly once and all
+// :77-78, and for 2-16 new tokens per sequence (pli_decode_fwd_multi) with the offset causal mask of :85-91, the tokens
+// of a q head served as extra rows of its KV group.  Addressing: ch07/paged_memory.py:38-48 pool layout, token t ->
+// page table[t / bs], slot t % bs (ceil-div rule, :54,:84-86).  HBM-bound: each K/V byte is read exactly once and all
 // q heads of a KV group are served from that one read.
 //
 //   decode_tma_kernel   bf16/f16, head_dim 64/128, page size 2^k in [8,256] (or contiguous): two producer warps stream
@@ -57,20 +58,24 @@ __global__ void __launch_bounds__(128) decode_simt_kernel(
     const T* __restrict__ q, const T* __restrict__ ks, const T* __restrict__ vs,
     const int32_t* __restrict__ table, const int32_t* __restrict__ seq_lens, int Hq, int Hkv, int D, int bs,
     int table_stride, int layer, int64_t qsb, int64_t qsh, int64_t s_page, int64_t s_layer, int64_t s_slot,
-    int64_t s_head, float scale, int S, float* __restrict__ o_part, float* __restrict__ lse_part) {
+    int64_t s_head, float scale, int S, float* __restrict__ o_part, float* __restrict__ lse_part, int q_len, int64_t qst) {
     __shared__ float sm_m[4], sm_d[4];
     extern __shared__ float sm_acc[];  // [4][D]
     const int s = blockIdx.x, h = blockIdx.y, b = blockIdx.z;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int hk = h / (Hq / Hkv);
     int t0, t1;
-    split_range(seq_lens[b], S, s, t0, t1);
+    const int L = seq_lens[b];
+    split_range(L, S, s, t0, t1);
+    // q_len > 1: h is a virtual head (q head * q_len + token index i), and token i sees keys j < L - (q_len - 1 - i)
+    // (ch02/cached_generation.py:85-91); a row left without keys in this split ends with m = -inf, den = 0
+    t1 = min(t1, L - (q_len - 1 - h % q_len));
 
     float qv[kDC], acc[kDC];
 #pragma unroll
     for (int c = 0; c < kDC; ++c) {
         const int d = lane + 32 * c;
-        qv[c] = d < D ? to_f32<T>(q[b * qsb + h * qsh + d]) : 0.f;
+        qv[c] = d < D ? to_f32<T>(q[b * qsb + (h / q_len) * qsh + (h % q_len) * qst + d]) : 0.f;
         acc[c] = 0.f;
     }
     float m = -INFINITY, dsum = 0.f;
@@ -281,7 +286,9 @@ struct DecodeTmaParams {
     float* lse_direct;
     int64_t osb, osh;
     int64_t qsb, qsh;
+    int64_t qst;                      // kMulti: token stride of q (row v of the problem is q head v / q_len, token v % q_len)
     int Hq, Hkv, G, bs, table_stride, layer, S, box_tokens, max_len;
+    int q_len;                        // kMulti: query tokens per sequence; Hq / G count virtual heads (q head * q_len + i)
     int bs_shift, box_shift;          // log2 of bs / box_tokens (both powers of two on this path)
     FastDiv fd_splits;                // division by S
     float scale_log2;
@@ -445,7 +452,12 @@ __device__ __forceinline__ void combine_unit(const DecodeTmaParams& p, uint8_t* 
     }
 }
 
-template <int kD, bool kBf16, bool kRows16>
+// kMulti: p.q_len query tokens per sequence (pli_decode_fwd_multi).  Row r of a unit is virtual head h_base + r, i.e.
+// token i = (h_base + r) % q_len of its q head, and sees keys j < seq_len - (q_len - 1 - i) (ch02/cached_generation.py:
+// 85-91).  Only the last q_len - 1 keys of a sequence differ between rows: that mask sits behind a warp-uniform test, so
+// interior stages run the one-token code.  A row can then see no key of a whole warp step or split (m = -inf): its
+// softmax update subtracts 0 instead of -inf, and the merges already weight a -inf state by 0.
+template <int kD, bool kBf16, bool kRows16, bool kMulti>
 __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid_constant__ CUtensorMap map_k,
                                                                     const __grid_constant__ CUtensorMap map_v,
                                                                     const __grid_constant__ DecodeTmaParams p) {
@@ -503,7 +515,7 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
     }
     // single-launch gather: this rank's kernel of step e has started, so its output buffer may be overwritten
     uint32_t step = 0;
-    if (p.gather.n > 0) {
+    if (!kMulti && p.gather.n > 0) {                                  // (no peer output with q_len > 1)
         step = *p.gather.epoch + 1u;
         if (blockIdx.x + blockIdx.y + blockIdx.z == 0 && warp == kConsumerWarps && lane < p.gather.n)
             st_release_sys(p.gather.ready[lane] + p.gather.rank, step);
@@ -617,7 +629,7 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
                 if (it == 0 && threadIdx.x == kConsumerWarps * 32) PLI_DECODE_TRACE(1);        // first stage's loads issued
             }
         }
-        if (p.gather.n > 0 && warp == kConsumerWarps) {
+        if (!kMulti && p.gather.n > 0 && warp == kConsumerWarps) {
             // every peer ready to receive step e?  (normally long true: they raised it when their kernels started)
             if (lane < p.gather.n &&
                 !wait_flag_reaches(p.gather.ready[p.gather.rank] + lane, step, p.gather.timeout_ns))
@@ -633,6 +645,15 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
         uint32_t qa[kD / 16][4];
         {
             const elem_t* qp = reinterpret_cast<const elem_t*>(p.q) + b * p.qsb;
+            // kMulti: row v of the unit is q head v / q_len, token v % q_len (two rows per thread: g0, g0 + 8)
+            int64_t q_row[2] = {0, 0};
+            if (kMulti) {
+#pragma unroll
+                for (int rr = 0; rr < 2; ++rr) {
+                    const int v = h_base + g0 + 8 * rr;
+                    q_row[rr] = (int64_t)(v / p.q_len) * p.qsh + (int64_t)(v % p.q_len) * p.qst;
+                }
+            }
 #pragma unroll
             for (int ks = 0; ks < kD / 16; ++ks) {
 #pragma unroll
@@ -641,7 +662,7 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
                     const int col = ks * 16 + qd + ((j & 2) ? 8 : 0);
                     uint32_t val = 0;
                     if (row < rows_here && (kRows16 || !(j & 1)))
-                        val = *reinterpret_cast<const uint32_t*>(qp + (h_base + row) * p.qsh + col);
+                        val = *reinterpret_cast<const uint32_t*>(qp + (kMulti ? q_row[j & 1] : (h_base + row) * p.qsh) + col);
                     qa[ks][j] = val;
                 }
             }
@@ -655,6 +676,11 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
         }
 #pragma unroll
         for (int n = 0; n < kNT; ++n) acc[n][0] = acc[n][1] = acc[n][2] = acc[n][3] = 0.f;
+        // kMulti: keys >= mask_from are hidden from some rows; row_cut[r] is the first key hidden from row g0 (+8)
+        const int mask_from = kMulti ? seq_len - p.q_len + 1 : 0;
+        int row_cut[kRowSlots];
+#pragma unroll
+        for (int r = 0; r < kRowSlots; ++r) row_cut[r] = kMulti ? mask_from + (hchunk * 16 + g0 + 8 * r) % p.q_len : 0;
 
         const uint32_t k_base = smem_u32(k_tiles), v_base = smem_u32(v_tiles);
         // ldmatrix lane roles: matrix id = lane / 8, row inside the matrix = lane % 8
@@ -693,11 +719,19 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
                             if (tk >= n_valid) sv[j] = -INFINITY;
                         }
                     }
+                    if (kMulti && tok_base + 16 > mask_from) {           // warp-uniform: the last q_len - 1 keys
+#pragma unroll
+                        for (int j = 0; j < 4; ++j) {
+                            const int tk = (j >> 1) * 8 + qd + (j & 1);
+                            if (tok_base + tk >= row_cut[r]) sv[j] = -INFINITY;
+                        }
+                    }
                     float mx = fmaxf(fmaxf(sv[0], sv[1]), fmaxf(sv[2], sv[3]));
                     mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 1));
                     mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
                     const float m_new = fmaxf(m_run[r], mx);
-                    const float ms = m_new * p.scale_log2;
+                    // (kMulti: a row with no key so far keeps m = -inf; subtracting 0 keeps alpha and p at 0, not NaN)
+                    const float ms = (kMulti && m_new == -INFINITY) ? 0.f : m_new * p.scale_log2;
                     const float alpha = ex2_approx(m_run[r] * p.scale_log2 - ms);   // m_run = -inf -> 0
                     float pv[4], psum = 0.f;
 #pragma unroll
@@ -841,7 +875,7 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
         }
         if (threadIdx.x == 0) PLI_DECODE_TRACE(4);               // output / partial written
         if (p.counters != nullptr && p.parts > 1 && p.cluster == 1) arrive_and_merge();   // (NULL: partials only)
-        if (p.gather.n > 0 && p.gather.cta_counter != nullptr) {
+        if (!kMulti && p.gather.n > 0 && p.gather.cta_counter != nullptr) {
             // ---- (option, off: see pli_decode_fwd_gather) the last CTA of the grid to get here publishes this rank's
             // slice and waits for the peers' ----
             named_bar_sync(1, kConsumerWarps * 32);              // every consumer thread's peer stores are issued
@@ -1107,9 +1141,9 @@ int make_kv_map(CUtensorMap* map, const void* base, int dtype, int D, int Hkv, b
     return PLI_OK;
 }
 
-template <int kD, bool kBf16, bool kRows16>
+template <int kD, bool kBf16, bool kRows16, bool kMulti>
 int launch_tma_t(const CUtensorMap& mk, const CUtensorMap& mv, DecodeTmaParams p, dim3 grid, cudaStream_t stream) {
-    auto kern = decode_tma_kernel<kD, kBf16, kRows16>;
+    auto kern = decode_tma_kernel<kD, kBf16, kRows16, kMulti>;
     constexpr int kTileBytes = (kD / 64) * kStageTokens * 128;
     const size_t merge_bytes = (size_t)(128 + 64 * (kD + 8)) * sizeof(float);
     size_t smem = (size_t)2 * kDecodeStages * kTileBytes + 2 * kDecodeStages * sizeof(uint64_t) + 24 + 1024;
@@ -1276,7 +1310,9 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
                         const int64_t kv_strides[4], float scale, int dtype, int num_splits, void* workspace,
                         size_t workspace_bytes, cudaStream_t stream, void* o_direct, float* lse_direct,
                         const int64_t* o_strides, bool* wrote_direct, const PeerScatter* peer = nullptr,
-                        const PeerGather* gather = nullptr) {
+                        const PeerGather* gather = nullptr, int q_len = 1, int64_t q_tok_stride = 0) {
+    // q_len > 1 (pli_decode_fwd_multi): Hq counts virtual heads (q head * q_len + token); q_strides are q's {batch, head}
+    // with q_tok_stride its token stride, o_strides are {batch, virtual head}
     const bool paged = block_table != nullptr;
     if (num_splits == 0) num_splits = pli_decode_num_splits(B, Hkv, max_seq_len);
     int rc = check_decode_args(q, k_store, v_store, seq_lens, B, Hq, Hkv, D, max_seq_len, block_size, paged, num_splits);
@@ -1290,7 +1326,8 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
     float* lse_part = o_part + (size_t)B * Hq * num_splits * D;
     const int G = Hq / Hkv;
 
-    if (tma_path_ok(q, k_store, v_store, D, dtype, block_size, paged, q_strides, kv_strides, scale)) {
+    if (tma_path_ok(q, k_store, v_store, D, dtype, block_size, paged, q_strides, kv_strides, scale) &&
+        (q_len == 1 || q_tok_stride % 2 == 0)) {
         const int box_tokens = paged ? (block_size < kStageTokens ? block_size : kStageTokens) : kStageTokens;
         // layers extent: the layer coordinate must be inside the tensor; layer+1 is a safe lower bound
         CUtensorMap mk, mv;
@@ -1343,6 +1380,7 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
         if (wrote_direct) *wrote_direct = direct || fused;
         p.qsb = q_strides[0];
         p.qsh = q_strides[1];
+        p.qst = q_tok_stride;
         p.Hq = Hq;
         p.Hkv = Hkv;
         p.G = G;
@@ -1352,6 +1390,7 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
         p.S = num_splits;
         p.box_tokens = box_tokens;
         p.max_len = max_seq_len;
+        p.q_len = q_len;
         p.bs_shift = ilog2(p.bs);
         p.box_shift = ilog2(box_tokens);
         p.fd_splits = make_fastdiv((uint32_t)num_splits);
@@ -1362,7 +1401,9 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
         dim3 grid(num_splits, Hkv * hchunks, B);
         const bool rows16 = G > 8;
         const bool bf16 = dtype == PLI_BF16;
-#define PLI_GO(DD, BF, R16) return launch_tma_t<DD, BF, R16>(mk, mv, p, grid, stream)
+#define PLI_GO(DD, BF, R16)                                                                                         \
+    return q_len > 1 ? launch_tma_t<DD, BF, R16, true>(mk, mv, p, grid, stream)                                   \
+                     : launch_tma_t<DD, BF, R16, false>(mk, mv, p, grid, stream)
         if (D == 128) {
             if (bf16) { if (rows16) PLI_GO(128, true, true); else PLI_GO(128, true, false); }
             else      { if (rows16) PLI_GO(128, false, true); else PLI_GO(128, false, false); }
@@ -1383,7 +1424,7 @@ static int splitkv_impl(const void* q, const void* k_store, const void* v_store,
     decode_simt_kernel<T, N><<<grid, 128, smem, stream>>>(                                                          \
         (const T*)q, (const T*)k_store, (const T*)v_store, block_table, seq_lens, Hq, Hkv, D, bs, table_stride,     \
         layer, q_strides[0], q_strides[1], kv_strides[0], kv_strides[1], kv_strides[2], kv_strides[3], scale,       \
-        num_splits, o_part, lse_part)
+        num_splits, o_part, lse_part, q_len, q_tok_stride)
 #define PLI_SIMT_D(T)                   \
     if (dc <= 1) PLI_SIMT(T, 1);        \
     else if (dc <= 2) PLI_SIMT(T, 2);   \
@@ -1615,6 +1656,46 @@ extern "C" int pli_decode_fwd(const void* q, const void* k_store, const void* v_
     if (rc) return rc;
     if (wrote_direct) return PLI_OK;
     return combine_impl(workspace, o, lse, B, Hq, D, num_splits, o_strides, dtype, stream, PeerScatter{});
+}
+
+// Split count of pli_decode_fwd_multi: the units of its TMA grid are (b, kv head, 16-row chunk of the G * q_len rows of a
+// KV head); with q_len == 1 this is pli_decode_num_splits(B, Hkv, max_seq_len), the choice of pli_decode_fwd.
+extern "C" int pli_decode_num_splits_multi(int B, int Hq, int Hkv, int q_len, int max_seq_len) {
+    if (Hq <= 0 || Hkv <= 0 || q_len <= 1) return pli_decode_num_splits(B, Hkv, max_seq_len);
+    return pli_decode_num_splits(B, Hkv * ((Hq / Hkv * q_len + 15) / 16), max_seq_len);
+}
+
+// q_len tokens per sequence: the q_len rows of a q head are virtual heads h * q_len + i of a (B, Hq * q_len, D) problem,
+// so every layer of the one-token launch (GQA map v / (G * q_len) == h / G, partials, LSE layout, fused / cluster /
+// two-pass merges) serves it unchanged; the kernels add the per-row causal limit and read row v of q at head v / q_len,
+// token v % q_len through q's own strides.  The output is written through the virtual head stride, hence o's layout rule.
+extern "C" int pli_decode_fwd_multi(const void* q, const void* k_store, const void* v_store, const int32_t* block_table,
+                                    const int32_t* seq_lens, void* o, float* lse, int B, int Hq, int Hkv, int q_len, int D,
+                                    int max_seq_len, int block_size, int table_stride, int layer, int64_t kv_extent,
+                                    const int64_t q_strides[3], const int64_t kv_strides[4], const int64_t o_strides[3],
+                                    float scale, int dtype, int num_splits, void* workspace, size_t workspace_bytes,
+                                    void* stream) {
+    if (!o || !q_strides || !o_strides || !kv_strides) return set_error(PLI_ERR_INVALID, "null output / stride argument");
+    if (q_len < 1) return set_error(PLI_ERR_INVALID, "q_len must be positive, got %d", q_len);
+    if (q_len > 16)
+        return set_error(PLI_ERR_UNSUPPORTED, "decode takes at most 16 query tokens per sequence, got %d "
+                                              "(use pli_prefill_paged_fwd / pli_prefill_fwd for longer chunks)", q_len);
+    if (Hq <= 0 || Hkv <= 0 || Hq % Hkv != 0) return set_error(PLI_ERR_INVALID, "Hq (%d) must be a positive multiple of Hkv (%d)", Hq, Hkv);
+    if (q_len > 1 && Hq > 1 && o_strides[1] != q_len * o_strides[2])
+        return set_error(PLI_ERR_INVALID, "o needs head stride == q_len * token stride (a (B, Hq, q_len, D) tensor "
+                                          "contiguous in its last three dimensions)");
+    if ((int64_t)Hq * q_len > 65535) return set_error(PLI_ERR_UNSUPPORTED, "Hq * q_len > 65535");
+    const int Hv = Hq * q_len;
+    const int64_t os[2] = {o_strides[0], q_len > 1 ? o_strides[2] : o_strides[1]};
+    if (num_splits == 0) num_splits = pli_decode_num_splits_multi(B, Hq, Hkv, q_len, max_seq_len);
+    bool wrote_direct = false;
+    int rc = splitkv_impl(q, k_store, v_store, block_table, seq_lens, B, Hv, Hkv, D, max_seq_len, block_size, table_stride,
+                          layer, kv_extent, q_strides, kv_strides, scale, dtype, num_splits, workspace, workspace_bytes,
+                          static_cast<cudaStream_t>(stream), o, lse, os, &wrote_direct, nullptr, nullptr, q_len,
+                          q_strides[2]);
+    if (rc) return rc;
+    if (wrote_direct) return PLI_OK;
+    return combine_impl(workspace, o, lse, B, Hv, D, num_splits, os, dtype, stream, PeerScatter{});
 }
 
 extern "C" int pli_kv_append(const void* k_new, const void* v_new, void* k_store, void* v_store, const int32_t* block_table,

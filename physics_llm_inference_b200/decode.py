@@ -19,7 +19,11 @@ from .kv_cache import KVCache, LayerKVCache
 from .paged_memory import PagedKVCache
 
 
-def decode_num_splits(B: int, Hkv: int, max_seq_len: int) -> int:
+def decode_num_splits(B: int, Hkv: int, max_seq_len: int, *, group: int = 1, q_len: int = 1) -> int:
+    """The library's split count; with q_len > 1 tokens per sequence (group = Hq / Hkv) the one pli_decode_fwd_multi
+    picks (pli_decode_num_splits_multi)."""
+    if q_len > 1:
+        return int(_lib.load().pli_decode_num_splits_multi(B, group * Hkv, Hkv, q_len, max_seq_len))
     return int(_lib.load().pli_decode_num_splits(B, Hkv, max_seq_len))
 
 
@@ -28,57 +32,16 @@ def decode_workspace(B: int, Hq: int, D: int, num_splits: int, device) -> torch.
     return torch.empty(nbytes // 4, dtype=torch.float32, device=device)
 
 
-def _prepare_decode(
-    q: torch.Tensor,
-    k_cache: torch.Tensor,
-    v_cache: torch.Tensor,
-    seq_lens,
-    *,
-    block_tables: torch.Tensor | None = None,
-    layer: int = 0,
-    scale: float | None = None,
-    return_lse: bool = False,
-    num_splits: int | None = None,
-    max_seq_len: int | None = None,
-    workspace: torch.Tensor | None = None,
-    out: torch.Tensor | None = None,
-    peer_out=None,
-    validate: bool = False,
-):
-    """Attention of one query token per sequence over cached K/V.
-
-    q         (B, Hq, 1, D) or (B, Hq, D)
-    seq_lens  int (one length for the whole batch, like the reference's caches) or (B,) int32 CUDA
-              tensor (ragged batch; no host sync is made to read it)
-    max_seq_len  host upper bound of seq_lens, used to pick the split count; defaults to the int
-              seq_lens, else the cache length (contiguous) / table width * page size (paged)
-    validate  opt-in host check (one sync) of seq_lens / block-table ranges; off by default (no host sync)
-    peer_out  a `sharding.PeerOutput`: q / caches are this rank's head shard; the kernel stores the shard's output
-              into EVERY rank's full (B_total, Hq_total, D) buffer over NVLink and the call returns that full tensor
-              once all ranks' slices have landed (fused all-gather, no NCCL call).
-    Returns o shaped like q (and lse (B, Hq) float32 when return_lse).
-    """
-    if not (q.is_cuda and k_cache.is_cuda and v_cache.is_cuda):
-        raise RuntimeError("flash_decode runs on CUDA tensors only: there is no CPU fallback for the decode path")
-    if q.dim() == 4:
-        if q.shape[2] != 1:
-            raise RuntimeError(f"decode takes one query token per sequence; got q {tuple(q.shape)} "
-                               "(use flash_attention_forward(..., causal=True) for chunks)")
-        q3 = q[:, :, 0, :]
-    elif q.dim() == 3:
-        q3 = q
-    else:
-        raise RuntimeError(f"q must be (B, Hq, 1, D) or (B, Hq, D); got {tuple(q.shape)}")
-    if q3.stride(-1) != 1:
-        q3 = q3.contiguous()
-    B, Hq, D = q3.shape
-    if not (q.dtype == k_cache.dtype == v_cache.dtype):
-        raise RuntimeError(f"q and the KV storage must share a dtype; got {q.dtype}, {k_cache.dtype}, {v_cache.dtype}")
+def _storage(q_dtype, B, Hq, D, k_cache, v_cache, seq_lens, block_tables, layer, max_seq_len, validate, scale,
+             q_len: int = 1):
+    """Checks and marshalling of the KV storage, lengths and scale shared by the one- and multi-token calls."""
+    lo = q_len if q_len > 1 else 0         # smallest length validate=True accepts
+    if not (q_dtype == k_cache.dtype == v_cache.dtype):
+        raise RuntimeError(f"q and the KV storage must share a dtype; got {q_dtype}, {k_cache.dtype}, {v_cache.dtype}")
     if k_cache.shape != v_cache.shape or k_cache.stride() != v_cache.stride():
         raise RuntimeError("k and v storage must have the same shape and strides")
     if k_cache.stride(-1) != 1:
         raise RuntimeError("KV storage must have a unit head_dim stride")
-    dev = q.device
     paged = block_tables is not None
     if paged:
         if k_cache.dim() != 5:
@@ -111,9 +74,10 @@ def _prepare_decode(
         raise RuntimeError(f"num_heads ({Hq}) must be a multiple of num_kv_heads ({Hkv})")
 
     if isinstance(seq_lens, int):
-        if not 0 < seq_lens <= cap:
-            raise ValueError(f"seq_len {seq_lens} outside (0, {cap}]")
-        lens = torch.full((B,), seq_lens, dtype=torch.int32, device=dev)
+        if not 0 < seq_lens <= cap or seq_lens < q_len:
+            raise ValueError(f"seq_len {seq_lens} outside ({lo}, {cap}]" if q_len == 1 else
+                             f"seq_len {seq_lens} outside [{q_len}, {cap}]: it counts the {q_len} new tokens")
+        lens = torch.full((B,), seq_lens, dtype=torch.int32, device=k_cache.device)
         if max_seq_len is None:
             max_seq_len = seq_lens
     else:
@@ -128,11 +92,70 @@ def _prepare_decode(
     if validate:        # opt-in, one synchronising copy: the device-side preconditions (see validate_paged_args)
         from .flash_attention import validate_paged_args
         if paged:
-            validate_paged_args(lens, block_tables, bs, P, min_len=0, max_seq_len=max_seq_len)
-        elif int(lens.max()) > max_seq_len or int(lens.min()) < 0:
-            raise ValueError(f"seq_lens outside [0, {max_seq_len}]")
+            validate_paged_args(lens, block_tables, bs, P, q_lens=q_len if q_len > 1 else None, min_len=0,
+                                max_seq_len=max_seq_len)
+        elif int(lens.max()) > max_seq_len or int(lens.min()) < lo:
+            raise ValueError(f"seq_lens outside [{lo}, {max_seq_len}]")
     if scale is None:
         scale = D ** -0.5
+    return Hkv, lens, block_tables, bs, kv_strides, kv_extent, table_ptr, tstride, max_seq_len, scale
+
+
+def _prepare_decode(
+    q: torch.Tensor,
+    k_cache: torch.Tensor,
+    v_cache: torch.Tensor,
+    seq_lens,
+    *,
+    block_tables: torch.Tensor | None = None,
+    layer: int = 0,
+    scale: float | None = None,
+    return_lse: bool = False,
+    num_splits: int | None = None,
+    max_seq_len: int | None = None,
+    workspace: torch.Tensor | None = None,
+    out: torch.Tensor | None = None,
+    peer_out=None,
+    validate: bool = False,
+):
+    """Attention of the newest query token(s) of each sequence over cached K/V.
+
+    q         (B, Hq, 1, D) or (B, Hq, D); or (B, Hq, Nq, D) with 2 <= Nq <= 16 new tokens per sequence (the verify
+              step of speculative decoding), attended in ONE launch: query i sees key j iff j <= i + seq_lens[b] - Nq
+              (ch02/cached_generation.py:85-91), so seq_lens counts the Nq new tokens and must be >= Nq
+    seq_lens  int (one length for the whole batch, like the reference's caches) or (B,) int32 CUDA
+              tensor (ragged batch; no host sync is made to read it)
+    max_seq_len  host upper bound of seq_lens, used to pick the split count; defaults to the int
+              seq_lens, else the cache length (contiguous) / table width * page size (paged)
+    validate  opt-in host check (one sync) of seq_lens / block-table ranges; off by default (no host sync)
+    peer_out  a `sharding.PeerOutput` (one query token only): q / caches are this rank's head shard; the kernel stores
+              the shard's output into EVERY rank's full (B_total, Hq_total, D) buffer over NVLink and the call returns
+              that full tensor once all ranks' slices have landed (fused all-gather, no NCCL call).
+    Returns o shaped like q (and lse (B, Hq) float32 when return_lse; (B, Hq, Nq) for Nq > 1).
+    """
+    if not (q.is_cuda and k_cache.is_cuda and v_cache.is_cuda):
+        raise RuntimeError("flash_decode runs on CUDA tensors only: there is no CPU fallback for the decode path")
+    if q.dim() == 4 and q.shape[2] != 1:
+        if not 2 <= q.shape[2] <= 16:
+            raise RuntimeError(f"decode takes 1 to 16 query tokens per sequence; got q {tuple(q.shape)} "
+                               "(use flash_attention_forward(..., causal=True) or flash_attention_paged for chunks)")
+        if peer_out is not None:
+            raise RuntimeError("peer_out takes one query token per sequence")
+        return _prepare_decode_multi(q, k_cache, v_cache, seq_lens, block_tables=block_tables, layer=layer, scale=scale,
+                                     return_lse=return_lse, num_splits=num_splits, max_seq_len=max_seq_len,
+                                     workspace=workspace, out=out, validate=validate)
+    if q.dim() == 4:
+        q3 = q[:, :, 0, :]
+    elif q.dim() == 3:
+        q3 = q
+    else:
+        raise RuntimeError(f"q must be (B, Hq, 1, D) or (B, Hq, D); got {tuple(q.shape)}")
+    if q3.stride(-1) != 1:
+        q3 = q3.contiguous()
+    B, Hq, D = q3.shape
+    dev = q.device
+    st = _storage(q.dtype, B, Hq, D, k_cache, v_cache, seq_lens, block_tables, layer, max_seq_len, validate, scale)
+    Hkv, lens, block_tables, bs, kv_strides, kv_extent, table_ptr, tstride, max_seq_len, scale = st
 
     lib = _lib.load()
     if num_splits is None:
@@ -186,14 +209,48 @@ def _prepare_decode(
     return _Prepared(dev, "", args, keep, out, lse, None, None, q.dim() == 4)
 
 
+def _prepare_decode_multi(q, k_cache, v_cache, seq_lens, *, block_tables, layer, scale, return_lse, num_splits,
+                          max_seq_len, workspace, out, validate):
+    """`_prepare_decode` for q (B, Hq, Nq, D), 2 <= Nq <= 16: one `pli_decode_fwd_multi` launch."""
+    B, Hq, Nq, D = q.shape
+    # q is read through its own strides (e.g. the (B, Nq, Hq, D).transpose(1, 2) view of a projection), never copied:
+    # a DecodePlan re-reads the caller's q at every call and graph replay
+    if q.stride(-1) != 1:
+        raise RuntimeError("q must have a unit head_dim stride")
+    dev = q.device
+    st = _storage(q.dtype, B, Hq, D, k_cache, v_cache, seq_lens, block_tables, layer, max_seq_len, validate, scale, Nq)
+    Hkv, lens, block_tables, bs, kv_strides, kv_extent, table_ptr, tstride, max_seq_len, scale = st
+    lib = _lib.load()
+    if num_splits is None:
+        num_splits = decode_num_splits(B, Hkv, max_seq_len, group=Hq // Hkv, q_len=Nq)
+    need = int(lib.pli_decode_workspace_bytes(B, Hq * Nq, D, num_splits))
+    if workspace is None:
+        workspace = torch.empty(need // 4, dtype=torch.float32, device=dev)
+    elif workspace.numel() * workspace.element_size() < need or not workspace.is_cuda:
+        raise RuntimeError(f"workspace too small: need {need} bytes")
+    if out is None:
+        out = torch.empty((B, Hq, Nq, D), dtype=q.dtype, device=dev)
+    elif out.shape != (B, Hq, Nq, D) or out.dtype != q.dtype or out.stride(-1) != 1 or \
+            (Hq > 1 and out.stride(1) != Nq * out.stride(2)):
+        raise RuntimeError(f"out must be ({B}, {Hq}, {Nq}, {D}), q's dtype, contiguous in its last three dimensions")
+    lse = torch.empty((B, Hq, Nq), dtype=torch.float32, device=dev) if return_lse else None
+    keep = (q, k_cache, v_cache, block_tables, lens, workspace, lse)
+    args = (q.data_ptr(), k_cache.data_ptr(), v_cache.data_ptr(), table_ptr, lens.data_ptr(), out.data_ptr(),
+            lse.data_ptr() if lse is not None else None, B, Hq, Hkv, Nq, D, max_seq_len, bs, tstride, layer, kv_extent,
+            _lib.i64(*q.stride()[:3]), _lib.i64(*kv_strides), _lib.i64(*out.stride()[:3]), float(scale),
+            _lib.dtype_code(q.dtype), num_splits, workspace.data_ptr(), workspace.numel() * workspace.element_size())
+    return _Prepared(dev, "", args, keep, out, lse, None, None, False, multi=True)
+
+
 class _Prepared:
     """A validated, marshalled decode call: everything but the stream."""
-    __slots__ = ("dev", "scatter", "args", "keep", "out", "lse", "peer_out", "ps", "four_d", "lib")
+    __slots__ = ("dev", "scatter", "args", "keep", "out", "lse", "peer_out", "ps", "four_d", "lib", "fwd")
 
-    def __init__(self, dev, scatter, args, keep, out, lse, peer_out, ps, four_d):
+    def __init__(self, dev, scatter, args, keep, out, lse, peer_out, ps, four_d, multi=False):
         self.dev, self.scatter, self.args, self.keep = dev, scatter, args, keep
         self.out, self.lse, self.peer_out, self.ps, self.four_d = out, lse, peer_out, ps, four_d
         self.lib = _lib.load()
+        self.fwd = self.lib.pli_decode_fwd_multi if multi else self.lib.pli_decode_fwd
 
     def launch(self):
         with _lib.on_device(self.dev):
@@ -209,7 +266,7 @@ class _Prepared:
                 # captured step copies into — the caller accounts for replays with peer_out.advance(n)
                 o = self.peer_out.finish_step(self.ps, stream)
             else:
-                _lib.check(self.lib.pli_decode_fwd(*self.args, stream))
+                _lib.check(self.fwd(*self.args, stream))
                 o = self.out.unsqueeze(2) if self.four_d else self.out
         return (o, self.lse) if self.lse is not None else o
 

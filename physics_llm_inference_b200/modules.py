@@ -86,10 +86,17 @@ class DecodeGraphRunner:
     Follows the reference's `CUDAGraphRunner` (ch08/cuda_graph.py:30-76): static input buffers, warm-up,
     capture, then `copy_ -> replay -> clone`.  Works because the C-ABI launches make no host allocation
     or synchronisation and read the sequence lengths from device memory.
+
+    tokens_per_step = k > 1: the step appends k tokens per sequence (q (B, Hq, k, D), k_new / v_new (B, k, Hkv, D))
+    and attends all k in one launch with the offset causal mask, e.g. the verify step of speculative decoding
+    (k - 1 draft tokens + 1); `run` returns (B, Hq, k, D).
     """
 
     def __init__(self, k_cache: torch.Tensor, v_cache: torch.Tensor, num_heads: int, *, block_tables=None, layer: int = 0,
-                 warmup_iterations: int = 3):
+                 warmup_iterations: int = 3, tokens_per_step: int = 1):
+        if not 1 <= tokens_per_step <= 16:
+            raise ValueError(f"tokens_per_step must be in [1, 16], got {tokens_per_step}")
+        self.tokens_per_step = n = tokens_per_step
         self.k_cache, self.v_cache = k_cache, v_cache
         self.block_tables, self.layer = block_tables, layer
         self.num_heads = num_heads
@@ -99,20 +106,22 @@ class DecodeGraphRunner:
         self.num_kv_heads, self.head_dim = k_cache.shape[-2], k_cache.shape[-1]
         self.capacity = block_tables.shape[1] * k_cache.shape[2] if paged else k_cache.shape[1]
         dev, dt = k_cache.device, k_cache.dtype
-        self.static_q = torch.zeros(self.batch, num_heads, 1, self.head_dim, device=dev, dtype=dt)
-        self.static_k = torch.zeros(self.batch, 1, self.num_kv_heads, self.head_dim, device=dev, dtype=dt)
+        self.static_q = torch.zeros(self.batch, num_heads, n, self.head_dim, device=dev, dtype=dt)
+        self.static_k = torch.zeros(self.batch, n, self.num_kv_heads, self.head_dim, device=dev, dtype=dt)
         self.static_v = torch.zeros_like(self.static_k)
         self.seq_lens = torch.zeros(self.batch, dtype=torch.int32, device=dev)   # lengths BEFORE the step
-        self.static_out = torch.empty(self.batch, num_heads, self.head_dim, device=dev, dtype=dt)
-        splits = decode_num_splits(self.batch, self.num_kv_heads, self.capacity)
+        out_shape = (self.batch, num_heads, self.head_dim) if n == 1 else (self.batch, num_heads, n, self.head_dim)
+        self.static_out = torch.empty(out_shape, device=dev, dtype=dt)
+        splits = decode_num_splits(self.batch, self.num_kv_heads, self.capacity, group=num_heads // self.num_kv_heads,
+                                   q_len=n)
         self.num_splits = splits
-        self.workspace = decode_workspace(self.batch, num_heads, self.head_dim, splits, dev)
+        self.workspace = decode_workspace(self.batch, num_heads * n, self.head_dim, splits, dev)
         self.graph: torch.cuda.CUDAGraph | None = None
 
     def _step(self):
         kv_append(self.k_cache, self.v_cache, self.static_k, self.static_v, self.seq_lens, block_tables=self.block_tables,
                   layer=self.layer)
-        self.seq_lens.add_(1)
+        self.seq_lens.add_(self.tokens_per_step)
         flash_decode(self.static_q, self.k_cache, self.v_cache, self.seq_lens, block_tables=self.block_tables,
                      layer=self.layer, num_splits=self.num_splits, max_seq_len=self.capacity, workspace=self.workspace,
                      out=self.static_out)
@@ -122,10 +131,13 @@ class DecodeGraphRunner:
         if not torch.cuda.is_available():
             return False
         start = seq_lens.to(device=self.seq_lens.device, dtype=torch.int32).clone()
-        # warm-up and capture append one token at position seq_lens[b]: it must exist (cache row / allocated page)
-        if int(start.max()) + 1 > self.capacity or int(start.min()) < 0:
+        # warm-up and capture append tokens_per_step tokens from position seq_lens[b]: they must exist (cache rows /
+        # allocated pages)
+        n = self.tokens_per_step
+        if int(start.max()) + n > self.capacity or int(start.min()) < 0:
             raise RuntimeError(f"cannot capture a decode step at lengths up to {int(start.max())}: the cache holds "
-                               f"{self.capacity} tokens per sequence and the step appends one")
+                               f"{self.capacity} tokens per sequence and the step appends "
+                               f"{'one' if n == 1 else n}")
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
