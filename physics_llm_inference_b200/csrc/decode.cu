@@ -731,8 +731,11 @@ __global__ void __launch_bounds__(kDecodeThreads) decode_tma_kernel(const __grid
                     mx = fmaxf(mx, __shfl_xor_sync(0xffffffffu, mx, 2));
                     const float m_new = fmaxf(m_run[r], mx);
                     // (kMulti: a row with no key so far keeps m = -inf; subtracting 0 keeps alpha and p at 0, not NaN)
-                    const float ms = (kMulti && m_new == -INFINITY) ? 0.f : m_new * p.scale_log2;
-                    const float alpha = ex2_approx(m_run[r] * p.scale_log2 - ms);   // m_run = -inf -> 0
+                    const float ms = (kMulti && m_new == -INFINITY) ? 0.f : __fmul_rn(m_new, p.scale_log2);
+                    // both products rounded (__fmul_rn is never fused): an FMA would keep the rounding residual of
+                    // m * scale_log2, making alpha != 1 while the maximum stands still, and the LSE drift by that
+                    // residual at every warp step (~3e-3 nats over 4096 keys with logits near 1000 nats)
+                    const float alpha = ex2_approx(__fmul_rn(m_run[r], p.scale_log2) - ms);   // m_run = -inf -> 0
                     float pv[4], psum = 0.f;
 #pragma unroll
                     for (int j = 0; j < 4; ++j) {
